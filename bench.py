@@ -2,6 +2,7 @@
 """bench.py -- MoE-layer forward tokens/s on B200 (BASELINE.json metric), one fused persistent kernel per step.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--sweeps a,b,..]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +23,12 @@ top-k checked against the CPU oracle on a sample of its tokens (outside any time
 `cpu_baseline` is a plain torch CPU forward of the same layer on the host cores (a reported baseline, not a target).
 `--impl reference` times that CPU implementation as the reference arm: the reference itself has no CPU path and cannot
 be built here (SURVEY.md section 8c), so the oracle port is the stated stand-in.
+
+`--steps K` is the number of steps of every timed loop of the headline configuration (device-resident and end to end).
+`--dump-outputs DIR` writes what the last device-resident timed step returned to its caller, the layer output, as
+float32 `DIR/out.npy` (`DIR/out_rank<r>.npy` per rank at N > 1); the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.  Above 64 MB for all ranks together a fixed, seeded sample of token rows
+is written instead (`dump_outputs`).
 """
 from __future__ import annotations
 
@@ -76,6 +83,26 @@ def make_inputs(cfg, nlx, rank):
     for i in range(nlx):  # per expert: keeps the fp32 temporary small at ffn 14336
         we[i] = torch.randn(2, cfg.P, cfg.H, generator=g).bfloat16()
     return x, wg, we
+
+
+DUMP_BUDGET_BYTES = 64 * 10 ** 6 - (1 << 16)   # all ranks' files together, .npy headers included
+
+
+def dump_outputs(directory, out, rank, world):
+    """This rank's layer output (a CPU tensor in the caller's [mini_batch, seq, d_model] shape) as float32
+    `out.npy` (`out_rank<r>.npy` at N > 1).  When the ranks' outputs together would exceed 64 MB, a fixed, seeded sample
+    of token rows (the same rows on every rank and in every run, in ascending order) is written as [rows, d_model]."""
+    import numpy as np
+
+    a = out.float().numpy()
+    flat = a.reshape(-1, a.shape[-1])
+    rows = DUMP_BUDGET_BYTES // world // (flat.shape[1] * flat.itemsize)
+    if rows < flat.shape[0]:
+        a = flat[np.sort(np.random.default_rng(0).choice(flat.shape[0], rows, replace=False))]
+    os.makedirs(directory, exist_ok=True)
+    path = os.path.join(directory, "out.npy" if world == 1 else f"out_rank{rank}.npy")
+    np.save(path, a)
+    return path
 
 
 def load_peaks():
@@ -357,8 +384,9 @@ def parity_check(env, ctx, cfg, xd, wgd, wed, n_tokens):
             "ok": bool(allr[:, 3].sum() == 0)}
 
 
-def run_config(env, name, steps, warmup, sampler, *, e2e=True, parity_tokens=0, out_in_slab=True):
-    """Measure one configuration; returns a dict with the device-resident and end-to-end numbers."""
+def run_config(env, name, steps, warmup, sampler, *, e2e=True, parity_tokens=0, out_in_slab=True, keep_output=False):
+    """Measure one configuration; returns a dict with the device-resident and end-to-end numbers (and, with
+    `keep_output`, a CPU copy of the last timed step's output as "output")."""
     from flashmoe_b200.runtime import MoEContext
 
     rank, world, dev = env.rank, env.world, env.dev
@@ -392,6 +420,8 @@ def run_config(env, name, steps, warmup, sampler, *, e2e=True, parity_tokens=0, 
     rows_total = env.sum_over_ranks(rows_exec)
     res = {"name": name, "ms": ms, "launches": launches, "rows_total": rows_total, "cfg": cfg, "nlx": nlx,
            "out_buffer": "symmetric accumulator (MoEContext.output_buffer)" if (out_in_slab and world > 1) else "caller tensor"}
+    if keep_output:  # copied now: the end-to-end arm and the parity forward below overwrite `out` at N > 1
+        res["output"] = out.cpu()
 
     if e2e:
         # end-to-end arm: host activations in, host output back, EVERY step; three steps in flight (public API:
@@ -399,7 +429,7 @@ def run_config(env, name, steps, warmup, sampler, *, e2e=True, parity_tokens=0, 
         depth = 3
         x_pins = [x.clone().pin_memory() for _ in range(depth)]
         out_pins = [torch.empty_like(x).pin_memory() for _ in range(depth)]
-        e2e_steps = max(6, min(steps, 60))
+        e2e_steps = steps
 
         def run_e2e(n):
             tickets = []
@@ -475,7 +505,13 @@ def main():
     ap.add_argument("--parity-tokens", type=int, default=int(os.environ.get("FM_BENCH_PARITY_TOKENS", "256")))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's layer output as float32 .npy files into DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path; the reference arm times a CPU sample whose size is set by timing")
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if world != args.gpus:
         if world == 1 and args.gpus > 1:
@@ -503,7 +539,10 @@ def main():
 
     name = args.config
     cfg = BASELINE_CONFIGS[name]
-    res = run_config(env, name, args.steps, args.warmup, sampler, e2e=not args.no_e2e, parity_tokens=args.parity_tokens)
+    res = run_config(env, name, args.steps, args.warmup, sampler, e2e=not args.no_e2e, parity_tokens=args.parity_tokens,
+                     keep_output=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res.pop("output"), rank, world)
     S, ms = cfg.S, res["ms"]
     roof = derived(res, world, peaks, args.steps)
     # DRAM traffic per launch comes from a committed `ncu --set full` capture; it describes one configuration at one N only

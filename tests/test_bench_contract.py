@@ -1,9 +1,12 @@
-"""bench.py's output contract on the CPU-only legs: the reference arm prints one JSON line with the agreed keys, and the
-multi-rank convention (only rank 0 works and prints) holds.  The GPU arm is exercised on the B200 box by the driver."""
+"""bench.py's output contract: on the CPU-only legs the reference arm prints one JSON line with the agreed keys, and the
+multi-rank convention (only rank 0 works and prints) holds; on the GPU, `--steps` sets the timed steps and
+`--dump-outputs` writes the layer output the timed path computed."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -153,3 +156,68 @@ def test_roofline_block_arithmetic():
     r8 = bench.derived({"cfg": cfg, "ms": 0.18, "rows_total": 8 * 8192, "nlx": 1}, 8, peaks, 20)
     assert abs(r8["nvlink_bytes_per_dir_per_gpu"] - 2.0 * 8192 * (7 / 8) * cfg.H * 2) < 1
     assert abs(r8["algorithmic_flops_per_launch"] - flops) < 1   # weak scaling: per-GPU work fixed
+
+
+def test_dump_outputs_whole_and_sampled(tmp_path):
+    """bench.dump_outputs: float32 in the caller's shape while all ranks' files fit in 64 MB; above that the same seeded
+    rows on every rank and in every run, within the budget."""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    g = torch.Generator().manual_seed(0)
+    small = torch.randn(1, 256, 64, generator=g).bfloat16()
+    path = bench.dump_outputs(str(tmp_path / "a"), small, 0, 1)
+    assert os.path.basename(path) == "out.npy"
+    a = np.load(path)
+    assert a.dtype == np.float32 and a.shape == (1, 256, 64) and (a == small.float().numpy()).all()
+
+    big = torch.randn(2, 8192, 1024, generator=g).bfloat16()   # 4 ranks x 64 MiB of float32 > 64 MB
+    paths = [bench.dump_outputs(str(tmp_path / "b"), big, r, 4) for r in range(4)]
+    assert [os.path.basename(p) for p in paths] == [f"out_rank{r}.npy" for r in range(4)]
+    assert sum(os.path.getsize(p) for p in paths) <= 64 * 10 ** 6
+    rows = bench.DUMP_BUDGET_BYTES // 4 // (1024 * 4)
+    idx = np.sort(np.random.default_rng(0).choice(2 * 8192, rows, replace=False))
+    b = np.load(paths[0])
+    assert b.dtype == np.float32 and b.shape == (rows, 1024)
+    assert (b == big.float().numpy().reshape(-1, 1024)[idx]).all()
+    again = bench.dump_outputs(str(tmp_path / "c"), big, 0, 4)
+    assert (np.load(again) == b).all()
+
+
+@pytest.mark.parametrize("args", [("--steps", "0"), ("--impl", "reference", "--dump-outputs", "unused")])
+def test_bench_rejects_arguments_it_cannot_honour(args, tmp_path):
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                         cwd=tmp_path, timeout=300)
+    assert res.returncode == 2 and "error" in res.stderr and not os.listdir(tmp_path)
+
+
+@pytest.mark.gpu
+def test_gpu_arm_steps_and_dumped_output(tmp_path):
+    """`--steps 3` runs three timed launches and three end-to-end steps; `--dump-outputs` writes config B's layer output
+    of the last timed step, which matches the CPU oracle on bench.py's own seeded inputs."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+    from oracle import moe_oracle as mo
+    from tests.util import check_output, run_oracle
+
+    out_dir = tmp_path / "dump"
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3",
+                          "--no-cpu-baseline", "--parity-tokens", "0", "--dump-outputs", str(out_dir)],
+                         capture_output=True, text=True, cwd=ROOT, timeout=600)
+    assert res.returncode == 0, res.stderr[-4000:]
+    d = json.loads([l for l in res.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 3 and d["gpu_launches"] == 3 and d["e2e"]["steps"] == 3
+    assert sorted(os.listdir(out_dir)) == ["out.npy"]
+    got = np.load(out_dir / "out.npy")
+    cfg = bench.BASELINE_CONFIGS["B"]
+    assert got.dtype == np.float32 and got.shape == (cfg.mini_batch, cfg.sequence_len, cfg.H)
+    x, wg, we = bench.make_inputs(cfg, cfg.E, 0)
+    ref = run_oracle(cfg, x, wg, we)
+    got_bits = mo.f32_to_bits(got.reshape(cfg.S, cfg.H))   # exact: the values are bf16
+    # the dump carries no routing tables: compare all rows the oracle does not flag as ambiguous
+    check_output(got_bits, ref.out, rows_ok=~ref.ambiguous, what="dumped output vs oracle")
