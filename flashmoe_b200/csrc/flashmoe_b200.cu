@@ -103,10 +103,7 @@ struct fm_ctx {
     int grid = 0;
     int tpc = 0;
     int TN0 = 0, TN1 = 0, num_pkts = 0, num_blocks = 0, total_items = 0;
-    int bn0 = 256, bn1 = 256, claim_ahead_kb = 16;
-    int dbg_flags = 0;
     bool coop = true;    // cooperative launch attribute (validates co-residency of the persistent grid)
-    int prefetch_kb = 0;
     bool pair = false;   // cta_group::2: two CTAs (one cluster) per 256-row tile
     uint32_t epoch = 0;
     unsigned long long bar_count = 0;
@@ -145,11 +142,6 @@ struct fm_ctx {
     bool dense = false;   // E == 1: GEMM0 reads x in place, no router GEMV, no dispatch copy (reference fffn.cuh:31-167)
     float* aux = nullptr; // is_training: [2][2E+1] {gML, gMeC, loss} by epoch parity
     const void* cached_x = nullptr;
-    int* recv_tok = nullptr;            // [nLx, pEC] slot -> token of the local packets (TMA gather4 source rows)
-    unsigned int* tok_rows = nullptr;   // [2, nLx, TCM]
-    bool gather = false;
-    const void* cached_xg = nullptr;
-    CUtensorMap tm_xg;
     bool tc_gate = false;               // router logits on the tensor cores (E <= 256)
     const void* cached_gx = nullptr;
     const void* cached_gw = nullptr;
@@ -221,6 +213,61 @@ int dev_alloc(T** p, size_t count, bool zero = true) {
     return FM_OK;
 }
 
+// The FFN work list: runs of work items (all tiles of one GEMM of one packet, or of a packet pair), claimed in this
+// order by the CTAs' schedulers, followed by a sentinel {kind -1, start = total items}.
+// Sources in the order own rank, rank+1, ... (local rows need no NVLink hop, so they are ready first).
+// With CTA pairs a work item is a 256-row tile made of two 128-row halves that share the B operand (same local expert):
+//   * world even and an odd number of row blocks per packet: halves = the SAME row block of the packets of two
+//     different source ranks ("cross-source pairing": no half is wasted -- with 128 experts on 8 GPUs every packet has
+//     exactly one);
+//   * otherwise:  halves = two consecutive row blocks of one packet (with an even number of row blocks this wastes
+//     nothing and keeps the local packets -- whose rows are ready first -- free of any remote dependency).
+// Orders:
+//   one rank:    all GEMM0, then all GEMM1 (measured best on config B);
+//   2-3 ranks:   GEMM0 local, GEMM0 remote, GEMM1 remote, GEMM1 local (the remote rows land while the local packets
+//                run; the outputs of remote packets cross NVLink as reductions and their done flags have a link round
+//                trip ahead of them, while the local adds, which nobody else waits for, come last);
+//   4+ ranks:    GEMM0 local, GEMM1 local, then the remote units with GEMM1 one source behind GEMM0 -- the local
+//                packets are the only work available until the remote rows have crossed NVLink (~50 us at 8 GPUs),
+//                and starting the remote units' GEMM1 early spreads the return traffic (reductions over NVLink at
+//                ~350 GB/s per GPU, which would otherwise pile up behind the last tiles) over the whole phase.
+std::vector<fm::TileBlock> build_work_list(int world, int rank, int nLx, int TCM, int TN0, int TN1, bool pair) {
+    const bool xpair = pair && world >= 2 && (world % 2) == 0 && (TCM % 2) == 1;
+    struct Unit { int pkt, pkt2; };
+    std::vector<Unit> loc, rem;   // units of this rank's own packets / of the other ranks' packets, in source order
+    for (int j = 0; j < world; j += xpair ? 2 : 1)
+        for (int le = 0; le < nLx; ++le) {
+            const Unit u = {((rank + j) % world) * nLx + le, xpair ? ((rank + j + 1) % world) * nLx + le : -1};
+            (j == 0 ? loc : rem).push_back(u);
+        }
+    std::vector<fm::TileBlock> blocks;
+    int start = 0;
+    auto push = [&](int kind, const Unit& u) {
+        blocks.push_back({kind, u.pkt, start, u.pkt2});
+        const int row_items = (pair && u.pkt2 < 0) ? (TCM + 1) / 2 : TCM;
+        start += row_items * (kind == 0 ? TN0 : TN1);
+    };
+    if (world >= 4) {
+        for (const Unit& u : loc) push(0, u);
+        for (const Unit& u : loc) push(1, u);
+        // remote units grouped by source rank (nLx units per source, or per source pair): GEMM1 one source behind GEMM0
+        const size_t per_src = (size_t)nLx;
+        for (size_t g0 = 0; g0 < rem.size(); g0 += per_src) {
+            for (size_t i = g0; i < std::min(g0 + per_src, rem.size()); ++i) push(0, rem[i]);
+            if (g0 >= per_src)
+                for (size_t i = g0 - per_src; i < g0; ++i) push(1, rem[i]);
+        }
+        for (size_t i = rem.size() >= per_src ? rem.size() - per_src : 0; i < rem.size(); ++i) push(1, rem[i]);
+    } else {
+        for (const Unit& u : loc) push(0, u);
+        for (const Unit& u : rem) push(0, u);
+        for (const Unit& u : rem) push(1, u);
+        for (const Unit& u : loc) push(1, u);
+    }
+    blocks.push_back({-1, 0, start, -1});
+    return blocks;
+}
+
 void set_peer_pointers(const fm_ctx* c, fm::FmParams& p) {
     for (int r = 0; r < c->d.world; ++r) {
         char* b = static_cast<char*>(c->peer_base[r]);
@@ -289,10 +336,6 @@ int launch(fm_ctx* c, const void* x, const void* gate_w, const void* expert_w, c
             c->cached_gw = gate_w;
         }
     }
-    if (c->gather && c->cached_xg != x) {   // x as [S, H] with a {64, 1} box: rows are picked one by one (TMA gather4)
-        if ((rc = make_tmap(&c->tm_xg, x, (uint64_t)d.S, d.H, 1))) return rc;
-        c->cached_xg = x;
-    }
     if (!c->tm_static_ready) {
         if (!c->dense && (rc = make_tmap(&c->tm_a0, static_cast<char*>(c->symm) + c->off_recv_x, (uint64_t)c->num_pkts * d.pEC, d.H,
                                          fm::BLOCK_M)))
@@ -306,22 +349,20 @@ int launch(fm_ctx* c, const void* x, const void* gate_w, const void* expert_w, c
         // of 2*P (resp. 2*H) rows is not expressible in 2-D, so rows are addressed as [nLx*2*P, H] / [nLx*2*H, P]:
         // expert i's W_up starts at row i*2*P, its W_down at row (i*2+1)*H of the [.,P] view.
         // in pair mode each CTA of the pair stages half of the B tile's rows
-        const uint32_t bdiv = c->pair ? 2u : 1u;
-        if ((rc = make_tmap(&c->tm_b0, expert_w, (uint64_t)nLx * 2 * d.P, d.H, (uint32_t)c->bn0 / bdiv))) return rc;
-        if ((rc = make_tmap(&c->tm_b1, expert_w, (uint64_t)nLx * 2 * d.H, d.P, (uint32_t)c->bn1 / bdiv))) return rc;
+        const uint32_t b_box = (uint32_t)fm::BLOCK_N / (c->pair ? 2u : 1u);
+        if ((rc = make_tmap(&c->tm_b0, expert_w, (uint64_t)nLx * 2 * d.P, d.H, b_box))) return rc;
+        if ((rc = make_tmap(&c->tm_b1, expert_w, (uint64_t)nLx * 2 * d.H, d.P, b_box))) return rc;
         c->cached_expert_w = expert_w;
     }
     fm::FmParams p;
     memset(&p, 0, sizeof(p));
     p.tm_a0 = c->tm_a0; p.tm_b0 = c->tm_b0; p.tm_a1 = c->tm_a1; p.tm_b1 = c->tm_b1;
-    if (c->gather) p.tm_xg = c->tm_xg;
     if (c->tc_gate) { p.tm_gx = c->tm_gx; p.tm_gw = c->tm_gw; }
     p.tc_gate = c->tc_gate ? 1 : 0;
     p.S = d.S; p.H = d.H; p.P = d.P; p.E = d.E; p.k = d.k; p.W = d.world; p.rank = d.rank; p.nLx = nLx;
     p.EC = d.EC; p.pEC = d.pEC; p.TCM = d.TCM; p.act = c->cfg.hidden_act;
     p.TN0 = c->TN0; p.TN1 = c->TN1; p.tpc = c->tpc; p.num_pkts = c->num_pkts; p.num_blocks = c->num_blocks;
     p.total_items = c->total_items;
-    p.bn[0] = c->bn0; p.bn[1] = c->bn1; p.claim_ahead_kb = c->claim_ahead_kb; p.dbg_flags = c->dbg_flags; p.prefetch_kb = c->prefetch_kb;
     // the epoch and the grid-barrier target advance only when the launch has been accepted (see below): a failed launch
     // must not leave the host ahead of the device counter and of the peers
     const uint32_t epoch = c->epoch + ((phase_mask & 1u) ? 1u : 0u);
@@ -357,9 +398,6 @@ int launch(fm_ctx* c, const void* x, const void* gate_w, const void* expert_w, c
     if (d.world == 1) p.peer_out_acc[0] = p.out;
     p.aux = c->aux;
     p.dense = c->dense ? 1 : 0;
-    p.gather = c->gather ? 1 : 0;
-    p.recv_tok = c->recv_tok;
-    p.tok_rows = c->tok_rows;
     p.dbg = c->dbg_dev;
     p.trace = c->trace_on ? c->trace : nullptr;
 
@@ -462,43 +500,31 @@ FM_API int fm_create(const fm_config_t* cfg, int rank, int world, int device, fm
     ctx->cfg = c;
     ctx->d = d;
     ctx->device = device;
-    // tuning knobs (tile widths of the two GEMMs, scheduler look-ahead); environment overrides are for experiments
+    // environment overrides of the defaults below: tests use them to cross-check the alternative paths
     auto env_int = [](const char* name, int dflt) {
         const char* v = getenv(name);
         return (v != nullptr && *v) ? atoi(v) : dflt;
     };
     ctx->grid = d.num_sms;  // one persistent CTA per SM; all co-resident (spin waits + grid barrier)
-    {
-        const char* v = getenv("FM_PAIR");
-        ctx->pair = (v != nullptr && *v) ? atoi(v) != 0 : true;   // default: CTA pairs (measured +9 % on config B)
-        // fused GEMM1 -> combine (REDG into the token's output row): only for k <= 2, where bf16 accumulation is
-        // order-independent (0 + a exact, a + b commutative) and therefore bit-identical to the deterministic gather;
-        // k > 2 keeps the gather so results do not depend on arrival order
-        const char* f = getenv("FM_FUSED_COMBINE");
-        ctx->fused = ((f != nullptr && *f) ? atoi(f) != 0 : true) && d.k <= 2;
-        ctx->dense = d.E == 1 && world == 1 && env_int("FM_DENSE_E1", 1) != 0;
-        // router logits by tcgen05.mma instead of the CUDA-core GEMV (2*S*H*E flops: 4.3 GFLOP per rank at E = 128,
-        // d_model 2048, 8192 tokens -- ~0.2 ms on the CUDA cores); one accumulator holds <= 256 experts
-        // Default: from 17 experts up.  Measured on one B200: E = 128, d_model 2048, 56 tokens per CTA: router 29 us instead
-        // of 433 us; E = 8, d_model 1024, 28 tokens per CTA (config B): a wash (the GEMV is latency-, not flop-bound there).
-        ctx->tc_gate = !ctx->dense && d.E <= 256 && env_int("FM_TC_GATE", d.E > 16 ? 1 : 0) != 0;
-        // TMA gather4 of local rows for tiles claimed before their copies landed: correct, but off by default -- measured on
-        // config B a gather tile takes 24 us instead of 6.6 (32 gather4 operations per k-block per CTA sustain only about
-        // one per 90 clocks), which costs far more than the ~5 us earlier start buys (160 vs 144 us per forward)
-        ctx->gather = !ctx->dense && env_int("FM_GATHER", 0) != 0;
-        if (ctx->pair && (ctx->grid & 1)) ctx->grid -= 1;  // CTA pairs need an even grid
-        ctx->d.grid = ctx->grid;
-    }
+    ctx->pair = env_int("FM_PAIR", 1) != 0;   // default: CTA pairs (measured +9 % on config B)
+    // fused GEMM1 -> combine (REDG into the token's output row): only for k <= 2, where bf16 accumulation is
+    // order-independent (0 + a exact, a + b commutative) and therefore bit-identical to the deterministic gather;
+    // k > 2 keeps the gather so results do not depend on arrival order
+    ctx->fused = env_int("FM_FUSED_COMBINE", 1) != 0 && d.k <= 2;
+    ctx->dense = d.E == 1 && world == 1 && env_int("FM_DENSE_E1", 1) != 0;
+    // router logits by tcgen05.mma instead of the CUDA-core GEMV (2*S*H*E flops: 4.3 GFLOP per rank at E = 128,
+    // d_model 2048, 8192 tokens -- ~0.2 ms on the CUDA cores); one accumulator holds <= 256 experts
+    // Default: from 17 experts up.  Measured on one B200: E = 128, d_model 2048, 56 tokens per CTA: router 29 us instead
+    // of 433 us; E = 8, d_model 1024, 28 tokens per CTA (config B): a wash (the GEMV is latency-, not flop-bound there).
+    ctx->tc_gate = !ctx->dense && d.E <= 256 && env_int("FM_TC_GATE", d.E > 16 ? 1 : 0) != 0;
+    if (ctx->pair && (ctx->grid & 1)) ctx->grid -= 1;  // CTA pairs need an even grid
+    ctx->d.grid = ctx->grid;
     ctx->tpc = ceil_div(d.S, ctx->grid);
     if ((long long)ctx->tpc * d.k > fm::G_SEL_MAX) {
         delete ctx;
         return fail(FM_EINVAL, "tokens-per-CTA * k = %d exceeds the router scratch (%d)", ctx->tpc * d.k, fm::G_SEL_MAX);
     }
     const int nLx = d.num_local_experts;
-    ctx->bn0 = env_int("FM_BN0", 256) == 128 ? 128 : 256;
-    ctx->bn1 = env_int("FM_BN1", 256) == 128 ? 128 : 256;
-    ctx->claim_ahead_kb = env_int("FM_CLAIM_AHEAD_KB", 16);   // measured on config B: 8 -> 144.5 us, 12 -> 142.3, 14 -> 140.6
-    ctx->dbg_flags = env_int("FM_DBG_FLAGS", 0);
     // The persistent grid spins on flags, counters and one grid barrier, so every CTA must be resident: the launch is
     // cooperative (the driver then refuses to start it unless the whole grid fits, also next to other work on the GPU).
     // One exception: Nsight Compute cannot replay a cooperative launch that also has cluster dimensions (the driver
@@ -526,86 +552,12 @@ FM_API int fm_create(const fm_config_t* cfg, int rank, int world, int device, fm
                         d.num_sms / 2, got, cudaGetErrorString(oe));
         }
     }
-    ctx->prefetch_kb = env_int("FM_PREFETCH_KB", 0);
-    if (ctx->prefetch_kb < 0) ctx->prefetch_kb = 0;
-    if (ctx->claim_ahead_kb < 0) ctx->claim_ahead_kb = 0;
-    ctx->TN0 = ceil_div(d.P, ctx->bn0);
-    ctx->TN1 = ceil_div(d.H, ctx->bn1);
+    ctx->TN0 = ceil_div(d.P, fm::BLOCK_N);
+    ctx->TN1 = ceil_div(d.H, fm::BLOCK_N);
     ctx->num_pkts = world * nLx;
-
-    // Work list.  Sources in the order own rank, rank+1, ... (local rows need no NVLink hop, so they are ready first).
-    // With CTA pairs a work item is a 256-row tile made of two 128-row halves that share the B operand (same local expert):
-    //   * world even: halves = the SAME row block of the packets of two different source ranks ("cross-source pairing":
-    //     no half is wasted when a packet has an odd number of row blocks -- with 128 experts on 8 GPUs every packet
-    //     has exactly one);
-    //   * otherwise:  halves = two consecutive row blocks of one packet.
-    // All GEMM0 blocks first, then the GEMM1 blocks (measured best on config B; FM_G1_LAG interleaves them with a lag).
-    // Cross-source pairing only pays when a packet has an ODD number of row blocks (otherwise pairing inside the packet
-    // wastes nothing and keeps the local packets -- whose rows are ready first -- free of any remote dependency).
-    const bool xpair = ctx->pair && world >= 2 && (world % 2) == 0 && (d.TCM % 2) == 1 && env_int("FM_XPAIR", 1) != 0;
-    struct Unit { int pkt, pkt2; bool local; };
-    std::vector<Unit> units;
-    if (xpair) {
-        for (int j = 0; j < world; j += 2)
-            for (int le = 0; le < nLx; ++le)
-                units.push_back({((rank + j) % world) * nLx + le, ((rank + j + 1) % world) * nLx + le, j == 0});
-    } else {
-        for (int j = 0; j < world; ++j)
-            for (int le = 0; le < nLx; ++le) units.push_back({((rank + j) % world) * nLx + le, -1, j == 0});
-    }
-    std::vector<fm::TileBlock> blocks;
-    int start = 0;
-    auto push = [&](int kind, const Unit& u) {
-        fm::TileBlock b;
-        b.kind = kind; b.pkt = u.pkt; b.start = start; b.pkt2 = u.pkt2;
-        blocks.push_back(b);
-        const int row_items = (ctx->pair && u.pkt2 < 0) ? (d.TCM + 1) / 2 : d.TCM;
-        start += row_items * (kind == 0 ? ctx->TN0 : ctx->TN1);
-    };
-    // GEMM0: local sources first (their rows are acknowledged first), then rank+1, rank+2, ...  GEMM1: REMOTE sources
-    // first, local last -- the outputs of remote packets cross NVLink as reductions and their done flags have a link round
-    // trip ahead of them, so they should not be what every rank finishes with; the local packets' adds are cheap and
-    // nobody but this rank waits for them.  FM_G1_LAG interleaves GEMM1 of a unit `lag` units after its GEMM0 instead.
-    std::vector<Unit> g1_units;
-    for (const Unit& u : units) if (!u.local) g1_units.push_back(u);
-    for (const Unit& u : units) if (u.local) g1_units.push_back(u);
-    // FM_G1_LAG: -1 (default) = the orders described here; n >= 1 = GEMM1 of a unit n units after its GEMM0.
-    //   one rank:    all GEMM0, then all GEMM1 (measured best on config B);
-    //   two ranks:   GEMM0 local, GEMM0 remote, GEMM1 remote, GEMM1 local (the remote rows land while the local packets
-    //                run; the local adds, which nobody else waits for, come last);
-    //   four+ ranks: GEMM0 local, GEMM1 local, then the remote units with GEMM1 one unit behind GEMM0 -- the local
-    //                packets are the only work available until the remote rows have crossed NVLink (~50 us at 8 GPUs),
-    //                and starting the remote units' GEMM1 early spreads the return traffic (reductions over NVLink at
-    //                ~350 GB/s per GPU, which would otherwise pile up behind the last tiles) over the whole phase.
-    const int lag = env_int("FM_G1_LAG", -1);
-    if (lag >= 1 && lag < (int)units.size()) {
-        for (size_t i = 0; i < units.size(); ++i) {
-            push(0, units[i]);
-            if ((int)i >= lag) push(1, units[i - lag]);
-        }
-        for (size_t i = units.size() - lag; i < units.size(); ++i) push(1, units[i]);
-    } else if (world >= 4 && lag < 0 && env_int("FM_LOCAL_FIRST", 1) != 0) {   // (0: the two-rank order, for A/B runs)
-        std::vector<Unit> loc, rem;
-        for (const Unit& u : units) (u.local ? loc : rem).push_back(u);
-        for (const Unit& u : loc) push(0, u);
-        for (const Unit& u : loc) push(1, u);
-        // remote units grouped by source rank (nLx units per source, or per source pair): GEMM1 one source behind GEMM0
-        const size_t per_src = xpair ? (size_t)nLx : (size_t)nLx;
-        for (size_t g0 = 0; g0 < rem.size(); g0 += per_src) {
-            for (size_t i = g0; i < std::min(g0 + per_src, rem.size()); ++i) push(0, rem[i]);
-            if (g0 >= per_src)
-                for (size_t i = g0 - per_src; i < g0; ++i) push(1, rem[i]);
-        }
-        for (size_t i = rem.size() >= per_src ? rem.size() - per_src : 0; i < rem.size(); ++i) push(1, rem[i]);
-    } else {
-        for (const Unit& u : units) push(0, u);
-        for (const Unit& u : g1_units) push(1, u);
-    }
-    ctx->num_blocks = (int)blocks.size();
-    ctx->total_items = start;
-    fm::TileBlock sentinel;
-    sentinel.kind = -1; sentinel.pkt = 0; sentinel.start = start; sentinel.pkt2 = -1;
-    blocks.push_back(sentinel);
+    std::vector<fm::TileBlock> blocks = build_work_list(world, rank, nLx, d.TCM, ctx->TN0, ctx->TN1, ctx->pair);
+    ctx->num_blocks = (int)blocks.size() - 1;
+    ctx->total_items = blocks.back().start;
 
 #define FM_TRY(expr)          \
     do {                      \
@@ -641,10 +593,6 @@ FM_API int fm_create(const fm_config_t* cfg, int rank, int world, int device, fm
     FM_TRY(dev_alloc(&ctx->hidden, (size_t)ctx->num_pkts * d.pEC * d.P));
     FM_TRY(dev_alloc(&ctx->trace, (size_t)ctx->grid * fm::TRACE_SLOTS));
     if (c.is_training) FM_TRY(dev_alloc(&ctx->aux, (size_t)2 * (2 * d.E + 1)));
-    if (ctx->gather) {
-        FM_TRY(dev_alloc(&ctx->recv_tok, (size_t)nLx * d.pEC));
-        FM_TRY(dev_alloc(&ctx->tok_rows, (size_t)2 * nLx * d.TCM));
-    }
 
     // symmetric slab: [recv_x | ret_y | recv_flag | ret_flag]  (reference heap + flags, bootstrap.cuh:348-362)
     size_t off = 0;
@@ -691,7 +639,7 @@ FM_API int fm_destroy(fm_ctx_t* ctx) {
         if (ctx->peer_opened[r] && ctx->peer_base[r] != nullptr) cudaIpcCloseMemHandle(ctx->peer_base[r]);
     void* bufs[] = {ctx->topk_idx, ctx->topk_w, ctx->mcw, ctx->slot, ctx->counts, ctx->gate_out, ctx->chunk_counts,
                     ctx->ctrl, ctx->g0_done, ctx->g1_done, ctx->pkt_done, ctx->recv_cnt, ctx->blocks, ctx->hidden, ctx->trace,
-                    ctx->aux, ctx->recv_tok, ctx->tok_rows};
+                    ctx->aux};
     for (void* b : bufs)
         if (b != nullptr) cudaFree(b);
     for (int i = 0; i < FM_HOST_SLOTS; ++i) {

@@ -36,10 +36,13 @@
 namespace fm {
 
 constexpr int BLOCK_M = 128;   // token rows per tile (= reference BLOCK_M)
-constexpr int BLOCK_N = 256;   // max output columns per tile (one tcgen05.mma N); per-GEMM width is p.bn[kind]
+constexpr int BLOCK_N = 256;   // output columns per tile (one tcgen05.mma N)
 constexpr int BLOCK_K = 64;    // 64 bf16 = 128 B = one swizzle row
 constexpr int UMMA_K = 16;
 constexpr int NSCHED = 4;
+// the scheduler claims the next tile when this many k-blocks of the current one remain (config B on one B200:
+// 8 -> 144.5 us per forward, 12 -> 142.3, 14 -> 140.6; 16 and larger alike)
+constexpr int CLAIM_AHEAD_KB = 16;
 constexpr int NUM_THREADS = 384;
 constexpr int NUM_WARPS = NUM_THREADS / 32;
 constexpr int EPI_WARP0 = 4;   // warps 4..11: warp % 4 selects the TMEM lane quarter, (warp - 4) / 4 the column half
@@ -113,18 +116,11 @@ struct FmParams {
     CUtensorMap tm_b0;  // expert_weights as [nLx*2*P, H]  box {64, 256}  (W_up rows)
     CUtensorMap tm_a1;  // hidden  as [W*nLx*pEC, P]  box {64, 128}
     CUtensorMap tm_b1;  // expert_weights as [nLx*2*H, P]  box {64, 256}  (W_down rows)
-    CUtensorMap tm_xg;  // x as [S, H], box {64, 1}: TMA gather4 of token rows for local packets (no dispatch copy needed)
     CUtensorMap tm_gx;  // router on tensor cores: x as [S, H], box {64, 32}
     CUtensorMap tm_gw;  // router on tensor cores: Wg_eff [E, H], box {64, E_pad} (CTA pair: {64, E_pad / 2})
     int tc_gate;        // 1 = logits by tcgen05.mma (E <= 256); 0 = register-blocked CUDA-core GEMV
     int S, H, P, E, k, W, rank, nLx, EC, pEC, TCM, act;
     int TN0, TN1, tpc, num_pkts, num_blocks, total_items;
-    int bn[2];          // tile width of GEMM0 / GEMM1 (128 or 256)
-    int claim_ahead_kb; // the scheduler claims the next tile when this many k-blocks of the current one remain
-    int prefetch_kb;    // L2 prefetch distance of the TMA producer in k-blocks (0 = off)
-    int dbg_flags;      // experiments only (results are garbage for bits 0-3): bit0 = skip all TMA loads, bit1 = skip MMA
-                        // issue, bit2 = skip the A loads, bit3 = skip the B loads, bit4 = partner CTA's producer also
-                        // arrives on the leader's `full` barrier (the round-1 handshake), bit5 = ignore BAR_DISP_DONE
     unsigned int epoch, phase_mask;
     unsigned long long bar_target, timeout_ns;
     const __nv_bfloat16 *x, *wg, *b_up, *b_down;
@@ -166,11 +162,6 @@ struct FmParams {
     __nv_bfloat16* peer_out_acc[FM_MAX_WORLD];
     // training mode (is_training = 1): [2][2E+1] f32 by epoch parity = {gML[E] mean gate probability per expert,
     // gMeC[E] mean routed fraction per expert, loss} (reference moe/gate.cuh:608-635,698-706,763-773); nullptr otherwise
-    // local packets (source = this rank): token of every slot, acknowledged BEFORE the row copies, so a GEMM0 tile
-    // claimed early can gather its A rows straight from x (TMA gather4) instead of waiting for the copies to land
-    int* recv_tok;             // [nLx, pEC] (local packets only, indexed by local expert)
-    unsigned int* tok_rows;    // [2, nLx, TCM] rows of block b whose token entry is written, by epoch parity
-    int gather;                // 0 = off
     float* aux;
     int dense;          // E == 1: no router GEMV, no dispatch copy; GEMM0 reads x in place (reference moe/fffn.cuh:31-167)
     DebugRecord* dbg;
@@ -832,31 +823,7 @@ __device__ __forceinline__ void dispatch_phase(const FmParams& p, uint8_t* smem,
             atomicAdd(a + 2 * E, __fdividef(me * ce, (float)E));
         }
     }
-    // Local packets first get their token table (slot -> token) and an acknowledgement of it: a GEMM0 tile claimed before
-    // the row copies below have landed gathers its rows from x by these indices (ffn_producer, TMA gather4).
     const unsigned int par = p.epoch & 1u;
-    if (p.gather) {
-        const int first_local = p.rank * p.nLx;
-        for (int i = tid; i < n_tok * k; i += DISP_THREADS) {
-            const int e = sel_e[i];
-            const int le = e - first_local;
-            if (le >= 0 && le < p.nLx) {
-                const int s = base_s[e] + rank_s[i];
-                if (s < p.EC) p.recv_tok[(size_t)le * p.pEC + s] = t0 + i / k;
-            }
-        }
-        disp_sync();
-        for (int le = tid; le < p.nLx; le += DISP_THREADS) {
-            const int e = first_local + le;
-            const int lo = base_s[e];
-            const int hi = min(lo + own_s[e], p.EC);
-            if (hi > lo) {
-                unsigned int* ctr = p.tok_rows + ((size_t)par * p.nLx + le) * p.TCM;
-                for (int b = lo / BLOCK_M; b <= (hi - 1) / BLOCK_M; ++b)
-                    red_release_gpu_add_u32(ctr + b, (unsigned int)(min(hi, (b + 1) * BLOCK_M) - max(lo, b * BLOCK_M)));
-            }
-        }
-    }
     // Row copies.
     //   * Rows for experts on THIS rank (warps 4-11): the chunk's token rows are contiguous in x, so one bulk load stages up
     //     to 128 KiB of them in shared memory (the first group was requested at the end of the router) and every kept
@@ -1052,9 +1019,9 @@ __device__ __forceinline__ void dispatch_phase(const FmParams& p, uint8_t* smem,
 
 // ============================================================================================================
 // Phase F: expert FFN.  Work items (global order, claimed with one atomic counter by the pair's scheduler warp):
-//   packets in the order (own rank first, then rank+1, ...); all GEMM0 blocks, then the GEMM1 blocks (host knob FM_G1_LAG
-//   interleaves them with a lag instead).  item -> (row-block pair m fastest, column tile n).  The item list is a static
-//   superset: row blocks beyond the packet's row count are skipped once the packet flag is known.  A GEMM1 tile waits for
+//   runs of all tiles of one GEMM of one packet, in the order of the host's build_work_list (own rank's packets first,
+//   then rank+1, ...).  item -> (row-block pair m fastest, column tile n).  The item list is a static superset: row
+//   blocks beyond the packet's row count are skipped once the packet flag is known.  A GEMM1 tile waits for
 //   g0_done[pkt][m] == TN0 (both row blocks of the pair).
 // ============================================================================================================
 struct TileInfo {     // 64 bytes, written by the (leader's) scheduler warp, read by producer / MMA / epilogue / publisher warps.
@@ -1062,8 +1029,8 @@ struct TileInfo {     // 64 bytes, written by the (leader's) scheduler warp, rea
     int kind;         // 0 GEMM0, 1 GEMM1, -1 stop
     int ntile;
     int le;           // local expert (both halves share it: same B operand)
-    int b_row;        // TMA row coordinate of the B tile (rank 1 of a pair: + bn/2)
-    int gather[2];    // GEMM0, local packet: 1 = this half's A rows are gathered from x (its row copies had not landed yet)
+    int b_row;        // TMA row coordinate of the B tile (rank 1 of a pair: + BLOCK_N/2)
+    int pad[2];       // keeps the struct at 4 x 16 bytes (ring slot size, DSMEM mirror)
     int pkt[2];       // local packet index src * nLx + le of each half
     int mblk[2];      // 128-row block of that packet
     int rows[2];      // valid rows of that block (0 = this half is idle)
@@ -1106,7 +1073,7 @@ __device__ __forceinline__ void ffn_scheduler(const FmParams& p, uint8_t* smem, 
         // The whole warp walks the claim loop in lock-step; lane h resolves the dependencies of half h of the item (the
         // two halves' flag / counter round trips overlap), lane 0 assembles and publishes the descriptor.
         int kind = -1, nt = 0, le = 0;
-        int h_pkt = 0, h_mb = 0, h_src = 0, h_rows = 0, h_cnt = 0, h_gather = 0;
+        int h_pkt = 0, h_mb = 0, h_src = 0, h_rows = 0, h_cnt = 0;
         for (;;) {
             int id = 0;
             if (lane == 0) id = (int)atomicAdd(p.claim, 1u);
@@ -1127,7 +1094,7 @@ __device__ __forceinline__ void ffn_scheduler(const FmParams& p, uint8_t* smem, 
             h_pkt = (h == 1 && cross) ? blk.pkt2 : blk.pkt;
             h_mb = cross ? m : (PAIR ? 2 * m + (h & 1) : m);
             h_src = h_pkt / p.nLx;
-            h_rows = 0; h_cnt = 0; h_gather = 0;
+            h_rows = 0; h_cnt = 0;
             if (h < nh && h_mb < p.TCM) {
                 const bool same_gpu = h_src == p.rank;   // flag and counters written from this GPU: gpu scope suffices
                 // wait for the packet (src, le): flag = {epoch, rows}  (reference subscriber.cuh:52-185)
@@ -1163,21 +1130,10 @@ __device__ __forceinline__ void ffn_scheduler(const FmParams& p, uint8_t* smem, 
                         const unsigned int* ctr = p.g0_done + (size_t)h_pkt * p.TCM + h_mb;
                         while (ld_acquire_gpu_u32(ctr) < (unsigned int)p.TN0)
                             g.tick(p.dbg, p.timeout_ns, FM_TRAP_G0_DONE, h_pkt, h_mb, 0);
-                        if (p.gather && p.fused && same_gpu && (p.phase_mask & 1u)) {
-                            // the block's GEMM0 tiles may all have run in gather mode, i.e. before its row copies and
-                            // routing records landed: the combine epilogue reads those records, so order behind their ack
-                            while (ld_acquire_gpu_u32(rctr) < (unsigned int)h_rows)
-                                g.tick(p.dbg, p.timeout_ns, FM_TRAP_RECV_ROWS, h_pkt, h_mb, h_rows);
-                        }
                     } else if ((p.phase_mask & 1u) && !p.dense) {  // GEMM0 needs the rows of this block to have landed (dispatch acks)
-                        // local packet: the token table of the block is acknowledged before its row copies -- if it is
-                        // complete while the rows are not, the producer gathers the rows from x itself (FM_GATHER=1)
-                        const unsigned int* tctr = (p.gather && same_gpu)
-                            ? p.tok_rows + ((size_t)(p.epoch & 1u) * p.nLx + le) * p.TCM + h_mb : nullptr;
                         for (;;) {
                             const unsigned int got = same_gpu ? ld_acquire_gpu_u32(rctr) : ld_acquire_sys_u32(rctr);
                             if (got >= (unsigned int)h_rows) break;
-                            if (tctr != nullptr && ld_acquire_gpu_u32(tctr) >= (unsigned int)h_rows) { h_gather = 1; break; }
                             g.tick(p.dbg, p.timeout_ns, FM_TRAP_RECV_ROWS, h_pkt, h_mb, h_rows);
                         }
                     }
@@ -1194,7 +1150,7 @@ __device__ __forceinline__ void ffn_scheduler(const FmParams& p, uint8_t* smem, 
         ti.kind = kind; ti.ntile = nt; ti.le = le;
         // expert_weights [nLx,2,P,H]: W_up(le) starts at row le*2*P of the [.,H] view; W_down(le) (the [P,H]
         // block flat-viewed as [H,P]) starts at row (le*2+1)*H of the [.,P] view.
-        ti.b_row = kind < 0 ? 0 : (kind == 0 ? le * 2 * p.P : (le * 2 + 1) * p.H) + nt * p.bn[kind];
+        ti.b_row = kind < 0 ? 0 : (kind == 0 ? le * 2 * p.P : (le * 2 + 1) * p.H) + nt * BLOCK_N;
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             ti.pkt[h] = __shfl_sync(0xffffffffu, h_pkt, h);
@@ -1202,7 +1158,6 @@ __device__ __forceinline__ void ffn_scheduler(const FmParams& p, uint8_t* smem, 
             ti.src[h] = __shfl_sync(0xffffffffu, h_src, h);
             ti.rows[h] = (kind >= 0 && h < nh) ? __shfl_sync(0xffffffffu, h_rows, h) : 0;
             ti.cnt[h] = __shfl_sync(0xffffffffu, h_cnt, h);
-            ti.gather[h] = (kind >= 0 && h < nh) ? __shfl_sync(0xffffffffu, h_gather, h) : 0;
         }
         if (lane == 0) {
             if (ti.kind >= 0 && n < 16) trace_stamp(p, 16 + n);
@@ -1243,35 +1198,19 @@ __device__ __forceinline__ void ffn_producer(const FmParams& p, uint8_t* smem, u
     int stage = 0, phase = 0, q = 0, qphase = 0;
     bool first = true, stamped = false;
     for (;;) {
-        int kind = -1, gather = 0, g_base = 0, g_rows = 0;
+        int kind = -1;
         TileInfo ti;
         if (lane == 0) {
             wait_sched_full<PAIR>(p, &sched_full[q], qphase, 300 + q);
             ti = ring[q];
             release_to_leader<PAIR>(&sched_empty[q], crank);
             kind = ti.kind;
-            const int hh0 = PAIR ? (int)crank : 0;
-            gather = ti.gather[hh0];
-            g_base = ti.le * p.pEC + ti.mblk[hh0] * BLOCK_M;   // this half's first slot in the local token table
-            g_rows = ti.rows[hh0];
         }
         kind = __shfl_sync(0xffffffffu, kind, 0);
         if (kind < 0) break;
-        gather = __shfl_sync(0xffffffffu, gather, 0);
-        // gather mode (GEMM0 tile of a local packet whose row copies have not landed): every lane owns four rows of the
-        // A tile and fetches them from x by token index, k-block by k-block (cp.async.bulk.tensor ... tile::gather4)
-        int4 tok = make_int4(0, 0, 0, 0);
-        if (gather) {
-            g_base = __shfl_sync(0xffffffffu, g_base, 0);
-            g_rows = __shfl_sync(0xffffffffu, g_rows, 0);
-            if (lane * 4 < g_rows) tok = ld_global_cg_i4(p.recv_tok + g_base + lane * 4);
-            if (lane * 4 + 1 >= g_rows) tok.y = 0;   // padding rows of the last block: any valid row (results are dropped)
-            if (lane * 4 + 2 >= g_rows) tok.z = 0;
-            if (lane * 4 + 3 >= g_rows) tok.w = 0;
-        }
         int nk = 0;
         if (lane == 0) {
-            if (first && (p.phase_mask & 1u) && !(p.dbg_flags & 32))   // the stage area doubles as the dispatch staging buffer
+            if (first && (p.phase_mask & 1u))   // the stage area doubles as the dispatch staging buffer
                 mbar_wait(&bars[BAR_DISP_DONE], 0, p.dbg, p.timeout_ns, FM_TRAP_MBAR_EMPTY, 901);
             first = false;
             fence_proxy_async_global();  // rows written by generic-proxy stores (peers / other SMs) -> TMA reads
@@ -1280,58 +1219,33 @@ __device__ __forceinline__ void ffn_producer(const FmParams& p, uint8_t* smem, u
         nk = __shfl_sync(0xffffffffu, nk, 0);
         const CUtensorMap* ta = kind == 0 ? &p.tm_a0 : &p.tm_a1;
         const CUtensorMap* tb = kind == 0 ? &p.tm_b0 : &p.tm_b1;
-        const int b_rows = p.bn[kind] / PC::B_ROWS_DIV;
-        const int take_at = min(nk - 1, max(0, nk - p.claim_ahead_kb));
+        constexpr int b_rows = BLOCK_N / PC::B_ROWS_DIV;
+        constexpr uint32_t tx = (uint32_t)A_STAGE_BYTES + (uint32_t)(b_rows * BLOCK_K * 2);
+        const int take_at = min(nk - 1, max(0, nk - CLAIM_AHEAD_KB));
         int a_row = 0, b_row = 0;
         if (lane == 0) {
             const int hh = PAIR ? (int)crank : 0;
             a_row = ti.pkt[hh] * p.pEC + ti.mblk[hh] * BLOCK_M;
             b_row = ti.b_row + (PAIR ? (int)crank * b_rows : 0);
-            const int pf = p.prefetch_kb;
-            if (pf > 0) {   // warm L2 for the k-blocks just beyond the smem pipeline
-                for (int kb = PC::STAGES; kb < min(nk, PC::STAGES + pf); ++kb) {
-                    tma_prefetch_l2_2d(ta, kb * BLOCK_K, a_row);
-                    tma_prefetch_l2_2d(tb, kb * BLOCK_K, b_row);
-                }
-            }
         }
         for (int kb = 0; kb < nk; ++kb) {
             uint8_t* sa = smem + stage * PC::STAGE_BYTES;
-            const bool ld_a = (p.dbg_flags & 5) == 0, ld_b = (p.dbg_flags & 9) == 0;   // experiments only
             if (lane == 0) {
-                const int pf = p.prefetch_kb;
-                if (pf > 0 && kb + PC::STAGES + pf < nk) {
-                    tma_prefetch_l2_2d(ta, (kb + PC::STAGES + pf) * BLOCK_K, a_row);
-                    tma_prefetch_l2_2d(tb, (kb + PC::STAGES + pf) * BLOCK_K, b_row);
-                }
                 if (kb == take_at && crank == 0) mbar_arrive(&prod_take[q]);  // lets the scheduler claim the next tile
                 mbar_wait(&empty[stage], phase ^ 1, p.dbg, p.timeout_ns, FM_TRAP_MBAR_EMPTY, stage);
-                const uint32_t tx = (ld_a ? (uint32_t)A_STAGE_BYTES : 0u) + (ld_b ? (uint32_t)(b_rows * BLOCK_K * 2) : 0u);
                 if (PAIR) {
                     // the leader's expect_tx covers both CTAs' bytes (every completion is credited to ITS barrier), so
                     // the partner's producer needs no arrival of its own: it only has to wait for its `empty` slot
-                    if (crank == 0) {
-                        if (tx) mbar_arrive_expect_tx(&full[stage], 2u * tx); else mbar_arrive(&full[stage]);
-                    } else if (p.dbg_flags & 17) {   // (bit 0: without loads nothing else keeps the partner in lock-step)
-                        mbar_arrive_cluster_plain(&full[stage], 0);
-                    }
+                    if (crank == 0) mbar_arrive_expect_tx(&full[stage], 2u * tx);
                     const uint32_t leader_full = mapa_shared(smem_u32(&full[stage]), 0);
-                    if (ld_a && !gather) tma_load_2d_pair(sa, ta, kb * BLOCK_K, a_row, leader_full);
-                    if (ld_b) tma_load_2d_pair(sa + A_STAGE_BYTES, tb, kb * BLOCK_K, b_row, leader_full);
+                    tma_load_2d_pair(sa, ta, kb * BLOCK_K, a_row, leader_full);
+                    tma_load_2d_pair(sa + A_STAGE_BYTES, tb, kb * BLOCK_K, b_row, leader_full);
                 } else {
-                    if (tx) mbar_arrive_expect_tx(&full[stage], tx); else mbar_arrive(&full[stage]);
-                    if (ld_a && !gather) tma_load_2d(sa, ta, kb * BLOCK_K, a_row, &full[stage]);
-                    if (ld_b) tma_load_2d(sa + A_STAGE_BYTES, tb, kb * BLOCK_K, b_row, &full[stage]);
+                    mbar_arrive_expect_tx(&full[stage], tx);
+                    tma_load_2d(sa, ta, kb * BLOCK_K, a_row, &full[stage]);
+                    tma_load_2d(sa + A_STAGE_BYTES, tb, kb * BLOCK_K, b_row, &full[stage]);
                 }
                 if (!stamped) { trace_stamp(p, 7); stamped = true; }   // first loads of the first tile issued
-            }
-            if (gather) {   // warp-uniform
-                __syncwarp();   // lane 0 has seen the stage empty
-                if (ld_a) {
-                    if (PAIR) tma_gather4_pair(sa + lane * 512, &p.tm_xg, kb * BLOCK_K, tok.x, tok.y, tok.z, tok.w,
-                                               mapa_shared(smem_u32(&full[stage]), 0));
-                    else tma_gather4(sa + lane * 512, &p.tm_xg, kb * BLOCK_K, tok.x, tok.y, tok.z, tok.w, &full[stage]);
-                }
             }
             if (++stage == PC::STAGES) { stage = 0; phase ^= 1; }
         }
@@ -1354,19 +1268,18 @@ __device__ __forceinline__ void ffn_mma(const FmParams& p, uint8_t* smem, uint64
     const int lane = threadIdx.x & 31;
     int stage = 0, phase = 0, q = 0, qphase = 0, as = 0, aphase = 0, nt = 0;
     for (;;) {
-        int kind = -1, nk = 0, bn = BLOCK_N;
+        int kind = -1, nk = 0;
         if (lane == 0) {
             mbar_wait(&sched_full[q], qphase, p.dbg, p.timeout_ns, FM_TRAP_MBAR_SCHED_FULL, q);
             kind = ring[q].kind;
             nk = kind < 0 ? 0 : (kind == 0 ? p.H : p.P) / BLOCK_K;
-            bn = kind < 0 ? BLOCK_N : p.bn[kind];
             mbar_arrive(&sched_empty[q]);
         }
         kind = __shfl_sync(0xffffffffu, kind, 0);
         if (++q == NSCHED) { q = 0; qphase ^= 1; }
         if (kind < 0) break;
         if (lane == 0) {
-            const uint32_t idesc = umma_idesc_bf16_f32(PAIR ? 2 * BLOCK_M : BLOCK_M, (uint32_t)bn);
+            const uint32_t idesc = umma_idesc_bf16_f32(PAIR ? 2 * BLOCK_M : BLOCK_M, (uint32_t)BLOCK_N);
             mbar_wait(&tmem_empty[as], aphase ^ 1, p.dbg, p.timeout_ns, FM_TRAP_MBAR_TMEM_EMPTY, as);
             tcgen05_fence_after();
             const uint32_t d_tmem = tmem_base + (uint32_t)as * BLOCK_N;
@@ -1379,7 +1292,6 @@ __device__ __forceinline__ void ffn_mma(const FmParams& p, uint8_t* smem, uint64
                 const uint64_t db = umma_smem_desc_sw128(sa + A_STAGE_BYTES);
 #pragma unroll
                 for (int kk = 0; kk < BLOCK_K / UMMA_K; ++kk) {
-                    if (p.dbg_flags & 2) break;   // experiment: no MMA, commits only
                     // +32 bytes per UMMA_K step inside the 128-byte swizzle row (address field is in 16-byte units)
                     if (PAIR) umma_bf16_ss_pair(d_tmem, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), idesc,
                                                 (kb | kk) != 0 ? 1u : 0u);
@@ -1517,8 +1429,7 @@ __device__ __forceinline__ void ffn_epilogue(const FmParams& p, uint8_t* smem, u
         if (++q == NSCHED) { q = 0; qphase ^= 1; }
         if (ti.kind < 0) break;
         const int N = ti.kind == 0 ? p.P : p.H;
-        const int bn = p.bn[ti.kind];
-        const int n0 = ti.ntile * bn;
+        const int n0 = ti.ntile * BLOCK_N;
         const int hh = PAIR ? (int)crank : 0;
         const int my_rows = ti.rows[hh], my_mblk = ti.mblk[hh], my_pkt = ti.pkt[hh], my_src = ti.src[hh];
         const __nv_bfloat16* bias = ti.kind == 0 ? (p.b_up ? p.b_up + (size_t)ti.le * p.P : nullptr)
@@ -1534,8 +1445,8 @@ __device__ __forceinline__ void ffn_epilogue(const FmParams& p, uint8_t* smem, u
         }
         // 64-column chunks of the tile that exist (N is a multiple of 64, not necessarily of the tile width), split
         // between the two warps of this lane quarter
-        const int per_half = bn / 128;
-        const int nvalid = my_rows > 0 ? min(bn / 64, (N - n0) / 64) : 0;
+        constexpr int per_half = BLOCK_N / 128;
+        const int nvalid = my_rows > 0 ? min(BLOCK_N / 64, (N - n0) / 64) : 0;
         const int c0 = min(chalf * per_half, nvalid), c1 = min(c0 + per_half, nvalid);
         // fused GEMM1 -> combine: this thread owns accumulator row (quarter*32 + lane); fetch that row's routing record
         const bool fuse = p.fused != 0 && ti.kind == 1;
@@ -1680,8 +1591,7 @@ __device__ __forceinline__ void ffn_setup(const FmParams& p, uint8_t* smem) {
         // arrival counts: full = leader's expect_tx; empty / tmem_full = one tcgen05.commit; tmem_empty = one lane per
         // epilogue warp (of both CTAs); pub_full = one lane per epilogue warp of this CTA; sched_empty = every ring reader
         const int nc = PAIR ? 2 : 1;
-        const int nfull = (PAIR && (p.dbg_flags & 17)) ? 2 : 1;
-        for (int i = 0; i < MAX_STAGES; ++i) { mbar_init(&bars[BAR_FULL + i], nfull); mbar_init(&bars[BAR_EMPTY + i], 1); }
+        for (int i = 0; i < MAX_STAGES; ++i) { mbar_init(&bars[BAR_FULL + i], 1); mbar_init(&bars[BAR_EMPTY + i], 1); }
         for (int i = 0; i < 2; ++i) {
             mbar_init(&bars[BAR_TMEM_FULL + i], 1);
             mbar_init(&bars[BAR_TMEM_EMPTY + i], NUM_EPI_WARPS * nc);
@@ -1717,12 +1627,13 @@ __device__ __forceinline__ void ffn_setup(const FmParams& p, uint8_t* smem) {
             const int local = id - blk.start;
             const bool cross = PAIR && blk.pkt2 >= 0;
             const int m_items = (PAIR && !cross) ? (p.TCM + 1) / 2 : p.TCM;
-            const int nt = local / m_items, le = blk.pkt % p.nLx, bn_w = p.bn[blk.kind];
+            const int nt = local / m_items, le = blk.pkt % p.nLx;
             const CUtensorMap* tb = blk.kind == 0 ? &p.tm_b0 : &p.tm_b1;
-            const int b0 = (blk.kind == 0 ? le * 2 * p.P : (le * 2 + 1) * p.H) + nt * bn_w;
-            const int nk_w = (blk.kind == 0 ? p.H : p.P) / BLOCK_K, step = PAIR ? bn_w / 2 : bn_w;
+            const int b0 = (blk.kind == 0 ? le * 2 * p.P : (le * 2 + 1) * p.H) + nt * BLOCK_N;
+            const int nk_w = (blk.kind == 0 ? p.H : p.P) / BLOCK_K;
+            constexpr int step = BLOCK_N / PipeCfg<PAIR>::B_ROWS_DIV;
             for (int kb = 0; kb < min(nk_w, PipeCfg<PAIR>::STAGES); ++kb)
-                for (int r = 0; r < bn_w; r += step) tma_prefetch_l2_2d(tb, kb * BLOCK_K, b0 + r);
+                for (int r = 0; r < BLOCK_N; r += step) tma_prefetch_l2_2d(tb, kb * BLOCK_K, b0 + r);
         }
     }
     if (warp == 2 && ((p.phase_mask & 2u) || p.tc_gate)) { if (PAIR) tmem_alloc_pair(tmem_ptr, TMEM_COLS); else tmem_alloc(tmem_ptr, TMEM_COLS); }
@@ -1931,10 +1842,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) fm_moe_forward_kernel(const __
             // peer can write them yet (a rank starts forward epoch+1 only after this launch has returned all its rows)
             unsigned int* next_rows = p.recv_rows + (size_t)((p.epoch + 1u) & 1u) * p.num_pkts * p.TCM;
             for (int i = tid; i < p.num_pkts * p.TCM; i += NUM_THREADS) next_rows[i] = 0u;
-            if (p.gather) {
-                unsigned int* next_tok = p.tok_rows + (size_t)((p.epoch + 1u) & 1u) * p.nLx * p.TCM;
-                for (int i = tid; i < p.nLx * p.TCM; i += NUM_THREADS) next_tok[i] = 0u;
-            }
             if (p.aux != nullptr) {   // the loss buffers of the next launch (reference clearState, moe.cuh:49-54)
                 float* next_aux = p.aux + (size_t)((p.epoch + 1u) & 1u) * (2 * p.E + 1);
                 for (int i = tid; i < 2 * p.E + 1; i += NUM_THREADS) next_aux[i] = 0.0f;

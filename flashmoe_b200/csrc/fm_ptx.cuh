@@ -361,26 +361,6 @@ __device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const void* tma
         ::"r"(smem_u32(smem_dst)), "l"(tmap), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
         : "memory");
 }
-// TMA gather: four arbitrary rows (r0..r3) of a 2-D tensor, `box` columns starting at column c0, land as four
-// consecutive 128-byte rows at smem_dst (tensor map encoded with box {64, 1}, 128-byte swizzle -- the swizzle is a
-// function of the shared-memory address, so a 512-byte aligned destination inside a tile keeps the tile's layout).
-__device__ __forceinline__ void tma_gather4(void* smem_dst, const void* tmap, int32_t c0, int32_t r0, int32_t r1, int32_t r2,
-                                            int32_t r3, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes.cta_group::1 "
-        "[%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-        ::"r"(smem_u32(smem_dst)), "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(r0), "r"(r1), "r"(r2), "r"(r3)
-        : "memory");
-}
-// CTA-pair form: issued by either CTA, completion bytes credited to the barrier at `bar_cluster_addr` (the leader's copy)
-__device__ __forceinline__ void tma_gather4_pair(void* smem_dst, const void* tmap, int32_t c0, int32_t r0, int32_t r1,
-                                                 int32_t r2, int32_t r3, uint32_t bar_cluster_addr) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes.cta_group::2 "
-        "[%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-        ::"r"(smem_u32(smem_dst)), "l"(tmap), "r"(bar_cluster_addr), "r"(c0), "r"(r0), "r"(r1), "r"(r2), "r"(r3)
-        : "memory");
-}
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result, uint32_t ncols) {  // same warp id in both CTAs
     asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
                  "r"(ncols)

@@ -104,7 +104,7 @@ def main():
         ctx.forward(x, wg, we, out=out)
     e1.record()
     ctx.synchronize()
-    print(f"=== {args.label or args.cfg}: {e0.elapsed_time(e1) / 20 * 1e3:.1f} us / forward (FM_DBG_FLAGS={os.environ.get('FM_DBG_FLAGS', '0')})")
+    print(f"=== {args.label or args.cfg}: {e0.elapsed_time(e1) / 20 * 1e3:.1f} us / forward")
     ctx.set_trace(True)
     ctx.forward(x, wg, we, out=out)
     ctx.synchronize()
